@@ -20,6 +20,8 @@ roofline: dominant kernel ntt_pass_v2_kernel; algorithmic bytes = 16 B per eleme
           from the committed ncu capture (profiles/ncu_traffic.json).
 cpu_baseline / --impl reference: the oracle's restatement of the reference CPU algorithm (one serial NTT per column,
           columns spread over all host threads, src/cs/implementations/utils.rs:295-304) on a bounded sample.
+--dump-outputs DIR: after the timed steps, a fixed sample of the batches as the last timed step left them (see dump_outputs),
+          so that two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import ctypes
@@ -36,6 +38,7 @@ SIZES = [20, 21, 22, 23, 24]
 BATCH_ELEMS_LOG = 27  # 1 GiB of u64 per size
 COSET = 7
 METRIC = "goldilocks_ntt_gelements_per_s"
+DUMP_SAMPLES = 1 << 19  # elements per size written by --dump-outputs: 5 sizes x 2^19 x 16 B = 40 MiB
 
 
 def load_peaks():
@@ -84,6 +87,21 @@ class ClockSampler(threading.Thread):
         s = sorted(self.samples)
         return {"sm_mhz": s[len(s) // 2] if s else None, "sm_max_mhz": self.max_mhz,
                 "reasons": [n for b, n in names.items() if self.reasons & b], "samples": len(s)}
+
+
+def dump_outputs(out_dir, data, rank, world):
+    """Writes out_dir/ntt_log<m>.npy (ntt_log<m>_rank<r>.npy on several GPUs) for every size m: the elements at fixed, seeded
+    positions of that size's batch, as float64 [samples, 2] = (high 32 bits, low 32 bits) of each u64 so that every value is
+    exact.  The positions depend only on m and the number of GPUs."""
+    import numpy as np
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    for m, t in data.items():
+        flat = t.view(-1)
+        idx = np.sort(np.random.default_rng(m).integers(0, flat.numel(), DUMP_SAMPLES // world))
+        v = flat[torch.from_numpy(idx).to(flat.device)].cpu().numpy().view(np.uint64)
+        pair = np.stack([v >> np.uint64(32), v & np.uint64(0xFFFFFFFF)], axis=1).astype(np.float64)
+        np.save(os.path.join(out_dir, "ntt_log%d%s.npy" % (m, "_rank%d" % rank if world > 1 else "")), pair)
 
 
 def run_reference(args, rank, world):
@@ -245,7 +263,10 @@ def main():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--prove-log-n", type=int, default=22, help="rows (log2) of the synthetic SHA-shaped proof; 0 disables")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="(b200 impl) write a fixed sample of the last timed step's outputs to DIR/*.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
 
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -321,6 +342,8 @@ def main():
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
         ms = float(t.item())
     value = world * elems_per_step / (ms * 1e-3) / 1e9
+    if args.dump_outputs:   # before the per-size breakdown below transforms the batches again
+        dump_outputs(args.dump_outputs, data, rank, world)
 
     # per-size breakdown (device time, CUDA events, same stream), after the headline region
     sweep = {}
